@@ -6,6 +6,7 @@ only, no per-step collective).
   python bench.py --gpus N --steps K --warmup W            # this repo (sm_100a engine through the public API)
   python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path (fp32 oracle on host cores)
   python bench.py --impl library --steps K ...             # torch fp16 library path (cuDNN + SDPA, CUDA graph) on the same GPU
+  python bench.py --steps K --dump-outputs DIR             # also writes the last timed frame's output to DIR/output.npy
 
 A "step" is one frame through StreamDiffusionPipeline.__call__.  `value` is timed on the device with the
 input frame already resident in HBM; `e2e` includes, every step, the pinned-host -> device copy of the frame
@@ -305,16 +306,27 @@ def main_gpu(args):
     import torch.distributed as dist
     os.environ.setdefault("B200SD_SYNTHETIC_WEIGHTS", "1")
     world_env = int(os.getenv("WORLD_SIZE", "1"))
-    nccl_glob = None
+    nccl_glob = log_dir = None
     nccl_env = {k: v for k, v in os.environ.items() if k.startswith("NCCL_DEBUG")}
     if world_env > 1 and os.environ.get("NCCL_DEBUG", "VERSION").upper() == "VERSION":   # unset, or the CUDA image's default
         # nobody asked for NCCL's log: keep stdout to the single JSON line, but still keep NCCL's own account of the job
         # (INFO level into per-process files, summarised in the line's "nccl" field).  A caller-provided NCCL_DEBUG is left
         # exactly as it is -- level and destination -- so a harness that reads NCCL's output from this process keeps seeing it.
-        os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
-        os.environ["NCCL_DEBUG"] = "INFO"
-        os.environ["NCCL_DEBUG_FILE"] = os.path.join(ROOT, "gpurun_out", f"nccl_n{world_env}_%h_%p.log")
-        nccl_glob = os.environ["NCCL_DEBUG_FILE"].replace("%h", "*").replace("%p", "*")
+        # The logs go to a directory of this launch under the temporary directory (the tree may be read-only).  Every rank
+        # derives the same name: the user id and the torchrun run id, or, without one, the launcher's pid (ranks started by one
+        # torchrun share it as their parent) and the rendezvous port.  Rank 0 removes the directory once it has summarised it.
+        import tempfile
+        launch = os.getenv("TORCHELASTIC_RUN_ID", "none")
+        if launch == "none":
+            launch = f"{os.getppid()}-{os.getenv('MASTER_PORT', '0')}"
+        log_dir = os.path.join(tempfile.gettempdir(), f"b200sd-bench-nccl-{os.getuid()}-{launch}")
+        os.makedirs(log_dir, exist_ok=True)
+        if os.stat(log_dir).st_uid != os.getuid():     # a directory of that name owned by someone else: NCCL's defaults
+            log_dir = None
+        else:
+            os.environ["NCCL_DEBUG"] = "INFO"
+            os.environ["NCCL_DEBUG_FILE"] = os.path.join(log_dir, f"nccl_n{world_env}_%h_%p.log")
+            nccl_glob = os.environ["NCCL_DEBUG_FILE"].replace("%h", "*").replace("%p", "*")
     os.environ["NVENC"] = "1"  # keep the output tensor in HBM (lib/pipeline.py:83,96)
     from ai_rtc_agent_b200.host import dist as bdist
     from ai_rtc_agent_b200.host.pipeline import StreamDiffusionPipeline
@@ -356,7 +368,8 @@ def main_gpu(args):
     torch.cuda.synchronize()
 
     def timed_device_loop(submit):
-        """K frames, device-timed on the current stream; `submit(i)` returns a ticket or None (stream-ordered call)."""
+        """K frames, device-timed on the current stream; `submit(i)` returns a ticket or None (stream-ordered call).
+        Returns the elapsed ms and the ticket of the last frame (None when `submit` returns no tickets)."""
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         last = collections.deque(maxlen=lanes)
@@ -368,7 +381,7 @@ def main_gpu(args):
             t.wait(cur)            # the closing event is ordered after the last frame of every lane
         e1.record()
         torch.cuda.synchronize()
-        return e0.elapsed_time(e1)
+        return e0.elapsed_time(e1), (last[-1] if last else None)
 
     # ---- device-resident throughput (value): frames already in HBM, public non-blocking entry, `lanes` frames in flight
     sampler = ClockSampler("GPU-" + str(torch.cuda.get_device_properties(dev).uuid)) if rank == 0 else None
@@ -377,15 +390,17 @@ def main_gpu(args):
     barrier()
     if sampler:
         sampler.start()
-    my_ms = timed_device_loop(lambda i: pipe.enqueue(ring_dev[(warm + i) % 64]))
+    my_ms, last_ticket = timed_device_loop(lambda i: pipe.enqueue(ring_dev[(warm + i) % 64]))
     barrier()
     clocks = sampler.stop() if sampler else None
+    # what the caller of the timed path received for its last frame: (1, 3, H, W) u8, stored as float32
+    dumped = {"output": last_ticket.result().float().cpu().numpy()} if args.dump_outputs and rank == 0 else None
     dev_ms = [r[0] for r in gather([my_ms])]
     ms_total = max(dev_ms)
     value = world * args.steps / (ms_total / 1000.0)
     # the same frames through the blocking call (one frame at a time, the reference's calling pattern): per-frame device latency
     barrier()
-    seq_ms = max(r[0] for r in gather([timed_device_loop(lambda i: (pipe(ring_dev[(warm + i) % 64]), None)[1])]))
+    seq_ms = max(r[0] for r in gather([timed_device_loop(lambda i: (pipe(ring_dev[(warm + i) % 64]), None)[1])[0]]))
     # ---- end to end through the public API with host buffers (e2e): every step copies its frame from pinned host memory and
     # reads its result back into pinned host memory; latency = submit -> result on the host.  Up to `lanes` frames are pending
     # (--e2e-pending): the next frame is submitted when the oldest has been retired, i.e. when its lane is free.  With lanes + 2
@@ -562,6 +577,14 @@ def main_gpu(args):
     if world > 1:
         line["nccl"] = dict(nccl_log_summary(nccl_glob) if nccl_glob else {"log": "NCCL_DEBUG* set by the caller, left untouched"},
                             caller_env=nccl_env, world_size=world, backend=dist.get_backend(), collectives_per_step=0)
+    if log_dir:
+        import shutil
+        shutil.rmtree(log_dir, ignore_errors=True)
+    if dumped:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in dumped.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
@@ -579,6 +602,11 @@ if __name__ == "__main__":
     ap.add_argument("--no-numa-pin", action="store_true")
     ap.add_argument("--e2e-pending", type=int, default=0, help="frames pending in the end-to-end loop (0 = frames_in_flight)")
     ap.add_argument("--workload", default="sd-turbo-512", choices=sorted(WORKLOADS))
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the output of the last timed step (rank 0: the (1,3,H,W) u8 frame the caller received, as float32) "
+                         "to DIR/output.npy; the inputs are seeded, so two builds can be compared output for output")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs is supported by --impl b200 only")
     select_workload(a.workload)
     sys.exit(main_reference(a) if a.impl == "reference" else (main_library(a) if a.impl == "library" else main_gpu(a)))

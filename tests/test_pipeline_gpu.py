@@ -280,7 +280,7 @@ def test_replicas_bit_identical_across_gpus_nccl(cuda):
     """Two ranks, NCCL weight broadcast from rank 0 (host/dist.py), identical frames in -> identical u8 out on both GPUs
     (all-gathered digests compared on every rank).  Needs 2 GPUs: skipped on a single-GPU box."""
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs 2 GPUs (gpurun --gpus 2)")
+        pytest.skip("needs 2 GPUs")
     port = 29600 + os.getpid() % 300
     cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node=2", "--master-addr", "127.0.0.1",
            "--master-port", str(port), os.path.join(ROOT, "tests", "replica_worker.py")]

@@ -1,19 +1,19 @@
 """Drop-in proof for the caller of the hot path (SURVEY.md 8 a-1 / f-2), CPU only.
 
-The reference's OWN, UNMODIFIED lib/tracks.py (/root/reference/lib/tracks.py:9-38) is loaded from the read-only reference
-checkout with `aiortc` stubbed (it is not installable offline) and driven by a fake source track.  It must run against this
-repo's pipeline call contract -- `pipeline(frame)` -- through warm-up, frame dropping and steady state, and this repo's
-non-blocking adapter (host/tracks.py) must make the same pipeline calls in the same order and return the same frames.
-/root/reference does not exist on the GPU box: those cases skip there; the adapter's own behaviour is tested everywhere."""
+The reference's OWN, UNMODIFIED lib/tracks.py (lib/tracks.py:9-38 of yondonfu/ai-rtc-agent) was run with `aiortc` stubbed
+(it is not installable offline) and driven by the fake source track below, against this repo's pipeline call contract --
+`pipeline(frame)` -- through warm-up, frame dropping and steady state.  tests/golden/make_tracks_golden.py recorded the frames
+it returned and the pipeline calls it made in tests/golden/reference_tracks.json; this repo's non-blocking adapter
+(host/tracks.py) must make the same pipeline calls in the same order and return the same frames."""
 import asyncio
-import importlib.util
+import json
 import os
-import sys
-import types
 
 import pytest
 
-REF_TRACKS = "/root/reference/lib/tracks.py"
+REF_TRACKS_GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_tracks.json")
+DROPS = [0, 1]    # DROP_FRAMES values the reference was recorded with
+RECV = 5          # recv() calls per recorded run
 
 
 class FakeSource:
@@ -58,21 +58,13 @@ class AsyncRecordingPipeline(RecordingPipeline):
         return Ticket(self(frame), polls=3)
 
 
-def _load_reference_tracks(monkeypatch):
-    if not os.path.exists(REF_TRACKS):
-        pytest.skip("reference checkout not present (GPU box)")
-    aiortc = types.ModuleType("aiortc")
-
-    class MediaStreamTrack:
-        def __init__(self):
-            self._ended = False
-
-    aiortc.MediaStreamTrack = MediaStreamTrack
-    monkeypatch.setitem(sys.modules, "aiortc", aiortc)
-    spec = importlib.util.spec_from_file_location("reference_lib_tracks", REF_TRACKS)
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)     # executes the reference's file as it is; nothing is copied into this repo
-    return mod
+def _reference_run(drop):
+    """(returned frames, pipeline calls, warm-up counter) of the reference's lib/tracks.py with DROP_FRAMES=drop."""
+    with open(REF_TRACKS_GOLDEN) as f:
+        gold = json.load(f)
+    assert gold["recv_calls"] == RECV
+    run = gold["runs"][str(drop)]
+    return [tuple(x) for x in run["out"]], [tuple(x) for x in run["calls"]], run["warmup_frame_idx"]
 
 
 def _drive(track, n):
@@ -81,24 +73,24 @@ def _drive(track, n):
     return asyncio.run(go())
 
 
-@pytest.mark.parametrize("drop", [0, 1])
+@pytest.mark.parametrize("drop", DROPS)
 def test_reference_tracks_py_runs_unchanged_and_adapter_matches_it(monkeypatch, drop):
     monkeypatch.delenv("WARMUP_FRAMES", raising=False)
     monkeypatch.setenv("DROP_FRAMES", str(drop))
-    ref_mod = _load_reference_tracks(monkeypatch)
-    ref_pipe, our_pipe = RecordingPipeline(), AsyncRecordingPipeline()
-    ref_track = ref_mod.VideoStreamTrack(FakeSource(), ref_pipe)
+    # the reference half is recorded data (tests/golden/reference_tracks.json, written by make_tracks_golden.py from the
+    # reference's unmodified lib/tracks.py); the two asserts on ref_* below pin that record, the others check this repo's adapter
+    ref_out, ref_calls, ref_warmup_idx = _reference_run(drop)
+    our_pipe = AsyncRecordingPipeline()
     from ai_rtc_agent_b200.host.tracks import VideoStreamTrack
     our_track = VideoStreamTrack(FakeSource(), our_pipe)
-    ref_out = _drive(ref_track, 5)
-    our_out = _drive(our_track, 5)
+    our_out = _drive(our_track, RECV)
     # warm-up: 10 frames through the pipeline, discarded (lib/tracks.py:21-25); then `drop` source frames skipped per output
     first = 10 + drop + 1
     assert ref_out[0] == ("processed", first)
-    assert [f[1] for f in ref_pipe.calls[:10]] == list(range(1, 11))
+    assert [f[1] for f in ref_calls[:10]] == list(range(1, 11))
     assert our_out == ref_out
-    assert our_pipe.calls == ref_pipe.calls
-    assert ref_track.warmup_frame_idx == our_track.warmup_frame_idx == 10
+    assert our_pipe.calls == ref_calls
+    assert ref_warmup_idx == our_track.warmup_frame_idx == 10
 
 
 def test_reference_tracks_py_imports_this_repos_pipeline_module(monkeypatch):

@@ -5,7 +5,7 @@ usage: python tools/summarize_launches.py gpurun_out/launches_<tag>.csv <tag>
 One frame = the launches from one `lcm_step_kernel`... boundary: we take the window between two consecutive
 `post_u8_kernel` launches (post_u8 is the last kernel of a frame).
 """
-import csv, json, re, sys, collections, shutil
+import csv, json, re, sys, collections
 
 src, tag = sys.argv[1], sys.argv[2]
 rows = collections.OrderedDict()
@@ -50,7 +50,10 @@ if "tconv_kernel" in agg:
     a = agg["tconv_kernel"]
     out += ["", f"tconv_kernel: {a['n']} launches/frame, DRAM traffic {(a['rd']+a['wr'])/1e6:.1f} MB/frame = {(a['rd']+a['wr'])/a['n']/1e6:.2f} MB per launch."]
 open(f"profiles/{tag}_launch_summary.md", "w").write("\n".join(out) + "\n")
-shutil.copy(src, f"profiles/{tag}_launches.csv")
+# the stored list ends with the summarised frame: the launches after it (the frame the capture stopped in) are dropped, which
+# keeps the file under 1 MB
+with open(src) as fi, open(f"profiles/{tag}_launches.csv", "w") as fo:
+    fo.writelines(l for l in fi if not l.startswith('"') or l.startswith('"ID"') or int(next(csv.reader([l]))[0]) <= ends[-1])
 json.dump({"dram_bytes_per_launch": per, "dram_bytes_per_frame": ig["rd"] + ig["wr"], "launches_per_frame": ig["n"],
            "note": f"igemm_kernel + igemm_pair_kernel, ncu dram__bytes_read.sum + dram__bytes_write.sum averaged over the launches of one SD-Turbo "
                    f"512x512 frame (profiles/{tag}_launches.csv)"}, open("profiles/igemm_traffic.json", "w"), indent=1)
