@@ -210,6 +210,14 @@ int b2sd_op_lcm_step(void* x, const void* eps, const void* noise, const float* c
                            do_add_noise, reinterpret_cast<cudaStream_t>(stream));
 }
 
+int b2sd_op_lcm_cfg_step(void* x, const void* eps, const void* noise, void* stock_noise, const float* coef, void* out_latent,
+                         int T, int hw, int do_add_noise, int cfg_type, float guidance_scale, float delta, void* stream) {
+    return lcm_cfg_step_launch(reinterpret_cast<__half*>(x), reinterpret_cast<const __half*>(eps),
+                               reinterpret_cast<const __half*>(noise), reinterpret_cast<__half*>(stock_noise), coef,
+                               reinterpret_cast<__half*>(out_latent), T, hw, do_add_noise, cfg_type, guidance_scale, delta,
+                               reinterpret_cast<cudaStream_t>(stream));
+}
+
 int b2sd_op_post_u8(const void* y_nhwc, int ldy, void* out_nchw_u8, int nb, int h, int w, void* stream) {
     return post_u8_launch(reinterpret_cast<const __half*>(y_nhwc), ldy, reinterpret_cast<uint8_t*>(out_nchw_u8), nb,
                           h, w, reinterpret_cast<cudaStream_t>(stream));

@@ -666,7 +666,8 @@ __global__ void __launch_bounds__(128) smallconv_kernel(SmallConvArgs a, int G) 
     for (int p = blockIdx.x * blockDim.x + threadIdx.x; p < npix; p += gridDim.x * blockDim.x) {
         const int xw = p % a.w_;
         const int yh = (p / a.w_) % a.h;
-        const int n = p / (a.w_ * a.h);
+        const int n_out = p / (a.w_ * a.h);
+        const int n = n_out < a.uc_rows ? n_out : n_out - a.uc_rows;   // source batch row
         float patch[K];
 #pragma unroll
         for (int tap = 0; tap < 9; ++tap) {
@@ -822,6 +823,94 @@ int lcm_step_launch(__half* x, const __half* eps, const __half* noise, const flo
                     int T, int hw, int do_add_noise, cudaStream_t s) {
     B2_LAUNCHED("lcm_step", launch_k(lcm_step_kernel, dim3((hw + 127) / 128), dim3(128), 0, s, 1, x, eps, noise, coef, out_latent, T, hw,
                                      do_add_noise));
+    return 0;
+}
+
+// ------------------------------------------------------------------------------------------ LCM step with residual CFG
+__device__ __forceinline__ void ld4h(const __half* p, float v[4]) {
+    const uint2 u = *reinterpret_cast<const uint2*>(p);
+    const __half2* h = reinterpret_cast<const __half2*>(&u);
+    *reinterpret_cast<float2*>(&v[0]) = __half22float2(h[0]);
+    *reinterpret_cast<float2*>(&v[2]) = __half22float2(h[1]);
+}
+__device__ __forceinline__ void st4h(__half* p, const float v[4]) {
+    uint2 u;
+    __half2* h = reinterpret_cast<__half2*>(&u);
+    h[0] = __floats2half2_rn(v[0], v[1]);
+    h[1] = __floats2half2_rn(v[2], v[3]);
+    *reinterpret_cast<uint2*>(p) = u;
+}
+
+// One thread per latent pixel walks the T slots in order, so the stock-noise shift (slot i reads slot i-1's old value) and
+// the latent-buffer re-noise (slot i gets slot i-1's x0) need no second pass.  eps rows: [uncond rows (u) | text rows (T)].
+__global__ void lcm_cfg_step_kernel(__half* __restrict__ x, const __half* __restrict__ eps, const __half* __restrict__ noise,
+                                    __half* __restrict__ stock, const float* __restrict__ coef, __half* __restrict__ out_latent,
+                                    int T, int hw, int do_add_noise, int cfg_type, float guidance, float delta) {
+    B2_PDL_ENTRY();
+    const int p = blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= hw) return;
+    const float* alpha = coef;
+    const float* beta = coef + T;
+    const float* c_skip = coef + 2 * T;
+    const float* c_out = coef + 3 * T;
+    const bool full = cfg_type == CFG_FULL;
+    const bool residual = cfg_type == CFG_SELF || cfg_type == CFG_INITIALIZE;   // eps_uncond = delta * stock noise
+    const int u = cfg_type == CFG_INITIALIZE ? 1 : (full ? T : 0);
+    float n0[4], prev_x0[4] = {0.f, 0.f, 0.f, 0.f}, prev_stock[4];
+    ld4h(noise + (long)p * 4, n0);
+    for (int i = 0; i < T; ++i) {
+        const long off = ((long)i * hw + p) * 4;
+        float xv[4], et[4], so[4], sv[4], eu[4], x0[4];
+        ld4h(x + off, xv);
+        ld4h(eps + off + (long)u * hw * 4, et);
+        ld4h(stock + off, so);
+        // predict_x0_batch (T > 1): stock = cat(init_noise[0:1], stock[:-1]);  initialize: stock[0] = eps of the uncond row
+#pragma unroll
+        for (int c = 0; c < 4; ++c) sv[c] = T > 1 ? (i == 0 ? n0[c] : prev_stock[c]) : so[c];
+        if (cfg_type == CFG_INITIALIZE && i == 0) ld4h(eps + (long)p * 4, sv);
+        if (full) ld4h(eps + off, eu);
+#pragma unroll
+        for (int c = 0; c < 4; ++c) {
+            if (!full) eu[c] = delta * sv[c];
+            const float pred = eu[c] + guidance * (et[c] - eu[c]);
+            x0[c] = c_out[i] * ((xv[c] - beta[i] * pred) / alpha[i]) + c_skip[i] * xv[c];
+            if (residual) {
+                // delta_x = scheduler_step(pred, beta * stock) * alpha_next / beta_next;  stock' = roll(init_noise, -1) + delta_x
+                const float sc = beta[i] * sv[c];
+                const float dx = c_out[i] * ((sc - beta[i] * pred) / alpha[i]) + c_skip[i] * sc;
+                const float an = i + 1 < T ? alpha[i + 1] : 1.f, bn = i + 1 < T ? beta[i + 1] : 1.f;
+                eu[c] = an * dx / bn;   // reuse: delta_x
+            }
+        }
+        if (residual) {
+            float nn[4];
+            if (i + 1 < T) ld4h(noise + off + (long)hw * 4, nn);
+            else { nn[0] = n0[0]; nn[1] = n0[1]; nn[2] = n0[2]; nn[3] = n0[3]; }
+#pragma unroll
+            for (int c = 0; c < 4; ++c) sv[c] = nn[c] + eu[c];
+        }
+        st4h(stock + off, sv);   // full: only the shift (the value never feeds the output)
+        if (i > 0) {
+            float nv[4] = {0.f, 0.f, 0.f, 0.f}, o[4];
+            if (do_add_noise) ld4h(noise + off, nv);
+#pragma unroll
+            for (int c = 0; c < 4; ++c) o[c] = alpha[i] * prev_x0[c] + beta[i] * nv[c];
+            st4h(x + off, o);
+        }
+#pragma unroll
+        for (int c = 0; c < 4; ++c) { prev_x0[c] = x0[c]; prev_stock[c] = so[c]; }
+    }
+    st4h(out_latent + (long)p * 4, prev_x0);
+}
+
+int lcm_cfg_step_launch(__half* x, const __half* eps, const __half* noise, __half* stock, const float* coef, __half* out_latent,
+                        int T, int hw, int do_add_noise, int cfg_type, float guidance, float delta, cudaStream_t s) {
+    if (cfg_type != CFG_SELF && cfg_type != CFG_INITIALIZE && cfg_type != CFG_FULL) {
+        b2_set_error("lcm_cfg_step: cfg_type %d is not self / initialize / full", cfg_type);
+        return -1;
+    }
+    B2_LAUNCHED("lcm_cfg_step", launch_k(lcm_cfg_step_kernel, dim3((hw + 127) / 128), dim3(128), 0, s, 1, x, eps, noise, stock, coef,
+                                         out_latent, T, hw, do_add_noise, cfg_type, guidance, delta));
     return 0;
 }
 

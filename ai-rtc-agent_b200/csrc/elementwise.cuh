@@ -46,6 +46,8 @@ struct SmallConvArgs {
     int nb, h, w_, cin, cout;
     int in_h, in_w;      // source extents (nearest resize when != h,w; VaeImageProcessor.resize)
     int flags;
+    int uc_rows;         // batch rows n < uc_rows read source row n, rows n >= uc_rows read row n - uc_rows:
+                         // the source is cat(x[0:uc_rows], x) (UNet input of classifier-free guidance); 0 = identity
 };
 int smallconv_launch(const SmallConvArgs& a, cudaStream_t s);
 // OIHW fp16 -> fp32 [cin*9][cout] (once, at load time)
@@ -57,6 +59,18 @@ int smallconv_prep_launch(const __half* w_oihw, float* wt, int cout, int cin, cu
 // x, eps: [T][hw][4] fp16; noise: [T][hw][4] fp16; coef: fp32 [4][T] = alpha, beta, c_skip, c_out.
 int lcm_step_launch(__half* x, const __half* eps, const __half* noise, const float* coef, __half* out_latent,
                     int T, int hw, int do_add_noise, cudaStream_t s);
+
+// The same with StreamDiffusion's classifier-free guidance (unet_step, guidance_scale > 1), one launch.  cfg_type is
+// B2SD_CFG_SELF / _INITIALIZE / _FULL; eps holds the UNet batch, uncond rows first: 0 (self), 1 (initialize) or T (full) of
+// them, then the T text rows.  stock: stock_noise [T][hw][4] fp16, read and updated in place.  Per slot i:
+//   s = stock after the T > 1 shift cat(noise[0:1], stock[:-1]); initialize: s[0] = eps[0]
+//   eps_uncond = full ? eps[i] : delta * s[i];  pred = eps_uncond + guidance * (eps_text[i] - eps_uncond)
+//   x0[i] = scheduler_step(pred, x[i]);  buffer update and out_latent as lcm_step
+//   self / initialize: stock[i] = noise[(i+1) % T] + scheduler_step(pred, beta[i] s[i]) * alpha[i+1] / beta[i+1]
+//   (alpha[T] = beta[T] = 1); full: stock[i] = s[i]
+enum : int { CFG_NONE = 0, CFG_SELF = 1, CFG_INITIALIZE = 2, CFG_FULL = 3 };
+int lcm_cfg_step_launch(__half* x, const __half* eps, const __half* noise, __half* stock, const float* coef, __half* out_latent,
+                        int T, int hw, int do_add_noise, int cfg_type, float guidance, float delta, cudaStream_t s);
 
 // Decoder tail + lib/pipeline.py:72-74 + image_utils.postprocess_image, on the fp16 grid:
 //   y16 (decoder conv out, fp16) -> y*2-1 -> /2+0.5 -> clamp(0,1) -> *255 -> clamp -> trunc to u8, NCHW

@@ -281,6 +281,16 @@ struct b2sd_engine {
     float* gn_ws = nullptr;    // GroupNorm chunk partials (shared: launches are stream-ordered)
     int* tile_counters = nullptr;
     float coef_host[4][64]{};
+    // classifier-free guidance (b2sd_set_guidance): requested settings, and the ones the current program was built with
+    struct Guidance { int cfg_type = B2SD_CFG_NONE; float scale = 1.f, delta = 1.f; };
+    Guidance guide_req, guide;     // guide.cfg_type == NONE unless guidance is active (cfg_type != none and scale > 1)
+    std::vector<__half> uncond_host;
+    int uc_rows = 0;               // unconditional rows in front of the T text rows of the UNet batch: 0, 1 (initialize), T (full)
+    int rows_cap = 0;              // UNet rows tsteps / temb* / gn_ws are sized for
+    __half* stock = nullptr;       // stock_noise NHWC [T][lh][lw][4]
+    __half* uctx = nullptr;        // unconditional prompt embeddings [ctx_tokens][D]
+    __half* ctx_rows = nullptr;    // guided batch with uncond rows: per-row prompt embeddings [B_u][Lpad][D] (zero padded)
+    int unet_rows() const { return cfg.batch + uc_rows; }
 
     unsigned long long* ln_stats = nullptr;   // slab of per-row LayerNorm statistics [rows][2] (see IgEpilogue::rowstat_out)
     size_t ln_stats_cap = 0, ln_stats_used = 0;   // in 64-bit words
@@ -834,19 +844,27 @@ int b2sd_engine::build_transformer(const std::string& p, const Act& x, int heads
     __half* wk2 = pack_rows(t + "attn2.k", {{t + "attn2.to_k.weight", head_perm(0)}}, D, s);
     __half* wv2 = pack_rows(t + "attn2.v", {{t + "attn2.to_v.weight", head_perm(0)}}, D, s);
     if (!wk2 || !wv2) return -1;
-    __half* kc = static_cast<__half*>(prog.alloc((size_t)L * Cp * 2));
     const int Lpad = 128 * ((L + 127) / 128);
-    __half* vct = static_cast<__half*>(prog.alloc((size_t)Cp * Lpad * 2));
+    // One prompt for every batch item, or (a guided batch with unconditional rows) one Lpad-row context per batch item: uncond
+    // or cond embeddings, zero padded, addressed by the attention's per-batch K / V^T strides.  Either way the K / V^T
+    // GEMMs run once per prompt (prog_prompt), not per frame.
+    const bool per_row = uc_rows > 0;
+    const int ctx_n = per_row ? B * Lpad : L;   // context rows of the K / V^T GEMMs
+    const int vt_ld2 = per_row ? B * Lpad : Lpad;
+    __half* kc = static_cast<__half*>(prog.alloc((size_t)ctx_n * Cp * 2));
+    __half* vct = static_cast<__half*>(prog.alloc((size_t)Cp * vt_ld2 * 2));
+    if (!kc || !vct) return -1;
     {
         allow_swap = false;
-        ActView ctxv{ctx, 1, 1, L, D, D};
+        const __half* cp = per_row ? ctx_rows : ctx;
+        ActView ctxv{cp, 1, 1, ctx_n, D, D};
         TRY(add_linear(prog_prompt, ctxv, wk2, Cp, D, nullptr, kc, Cp, nullptr, 0));
         ActView wvv{wv2, 1, 1, Cp, D, D};
         IgemmDesc d{};
         d.nseg = 1; d.src[0] = wvv; d.ntap[0] = 1;
-        d.w = ctx; d.w_rows = L; d.w_ld = D; d.stride = 1;
+        d.w = cp; d.w_rows = ctx_n; d.w_ld = D; d.stride = 1;
         d.Nb = 1; d.Ho = 1; d.Wo = Cp;
-        d.epi.out = vct; d.epi.ldc = Lpad; d.epi.acc_scale = 1.f; d.epi.res_scale = 1.f; d.epi.n_valid = L;
+        d.epi.out = vct; d.epi.ldc = vt_ld2; d.epi.acc_scale = 1.f; d.epi.res_scale = 1.f; d.epi.n_valid = ctx_n;
         TRY(add_igemm(prog_prompt, d));
         allow_swap = true;
     }
@@ -867,8 +885,8 @@ int b2sd_engine::build_transformer(const std::string& p, const Act& x, int heads
     {
         AttnDesc a{};
         a.q = q2.p; a.ldq = Cp;
-        a.k = kc; a.ldk = Cp; a.k_bstride = 0; a.k_rows = L;
-        a.vt = vct; a.ldvt = Lpad; a.vt_bstride = 0; a.vt_cols = L;
+        a.k = kc; a.ldk = Cp; a.k_bstride = per_row ? Lpad : 0; a.k_rows = ctx_n;
+        a.vt = vct; a.ldvt = vt_ld2; a.vt_bstride = per_row ? Lpad : 0; a.vt_cols = ctx_n;
         a.out = ao2.p; a.ldo = C;
         a.nb = B; a.heads = heads; a.sq = HW; a.skv = L; a.d_real = d_real; a.dp = dp;
         AttnPlan plan;
@@ -940,7 +958,7 @@ int b2sd_engine::build_program(cudaStream_t s) {
     taps.clear();
     launches = 0;
     drop_graphs();
-    const int B = cfg.batch, H = cfg.height, W = cfg.width;
+    const int T = cfg.batch, B = unet_rows(), H = cfg.height, W = cfg.width;   // B: UNet batch (T + unconditional rows)
     const int* ch = cfg.block_out_channels;
     const int nlev = 4;
     {
@@ -956,6 +974,20 @@ int b2sd_engine::build_program(cudaStream_t s) {
         ln_stats_used = 0;
         ln_stats = static_cast<unsigned long long*>(prog.alloc(ln_stats_cap * sizeof(unsigned long long)));
         if (!ln_stats) return -1;
+    }
+    ctx_rows = nullptr;
+    if (uc_rows > 0) {
+        // per-row prompt contexts of the guided batch, refreshed from uctx / ctx by the prompt program (b2sd_set_prompt_embeds)
+        const int L = cfg.ctx_tokens, D = cfg.cross_attention_dim, Lpad = 128 * ((L + 127) / 128);
+        ctx_rows = static_cast<__half*>(prog.alloc((size_t)B * Lpad * D * 2));
+        if (!ctx_rows) return -1;
+        CUDA_OK(cudaMemsetAsync(ctx_rows, 0, (size_t)B * Lpad * D * 2, s));   // padding rows: K = V = 0, masked by skv
+        __half* dst = ctx_rows; const __half* cond = ctx; const __half* unc = uctx; const int ucr = uc_rows;
+        prog_prompt.push_back(Op([=](cudaStream_t st) {
+            for (int r = 0; r < B; ++r)
+                if (cudaMemcpyAsync(dst + (size_t)r * Lpad * D, r < ucr ? unc : cond, (size_t)L * D * 2, cudaMemcpyDeviceToDevice, st) !=
+                    cudaSuccess) { b2_set_error("copy of the per-row prompt contexts failed"); return -1; }
+            return 0; }, "ctx rows"));
     }
 
     allow_swap = false;
@@ -1009,6 +1041,7 @@ int b2sd_engine::build_program(cudaStream_t s) {
         if (!a.wt) return -1;
         a.x = x_in.p; a.bias = vec({"conv_in.bias"});
         a.y = h.p; a.ldy = h.ld; a.nb = B; a.h = lh; a.w_ = lw; a.cin = 4; a.cout = ch[0]; a.in_h = lh; a.in_w = lw;
+        a.uc_rows = uc_rows;   // UNet input = cat(x[0:uc_rows], x): gathered here, never copied
         if (!a.bias) return -1;
         ++launches;
         prog_frame.push_back(Op([a](cudaStream_t st) { return smallconv_launch(a, st); }, "smallconv"));
@@ -1080,12 +1113,23 @@ int b2sd_engine::build_program(cudaStream_t s) {
     Act x0 = new_act(1, lh, lw, 4);
     {
         __half* xp = x_in.p; const __half* ep = eps.p; const __half* np_ = noise; const float* cf = coef; __half* op = x0.p;
-        const int T = B, hw = lh * lw, dan = cfg.do_add_noise;
+        const int hw = lh * lw, dan = cfg.do_add_noise;
         ++launches;
-        prog_frame.push_back(Op([=](cudaStream_t st) { return lcm_step_launch(xp, ep, np_, cf, op, T, hw, dan, st); }, "lcm_step"));
+        if (guide.cfg_type == B2SD_CFG_NONE) {
+            prog_frame.push_back(Op([=](cudaStream_t st) { return lcm_step_launch(xp, ep, np_, cf, op, T, hw, dan, st); }, "lcm_step"));
+        } else {
+            __half* sp = stock; const int ct = guide.cfg_type; const float g = guide.scale, dl = guide.delta;
+            prog_frame.push_back(Op([=](cudaStream_t st) { return lcm_cfg_step_launch(xp, ep, np_, sp, cf, op, T, hw, dan, ct, g, dl, st); },
+                                    "lcm_cfg_step"));
+        }
         idx_unet_end = prog_frame.size();
     }
     taps["x0"] = x0;
+    {
+        Act sn;
+        sn.p = stock; sn.n = T; sn.h = lh; sn.w = lw; sn.c = 4; sn.ld = 4;
+        taps["stock_noise"] = sn;
+    }
     allow_swap = false;
     // ================= TAESD decoder (DecoderTiny) =================
     Act dcur = new_act(1, lh, lw, 64);
@@ -1145,6 +1189,7 @@ int b2sd_engine::build_program(cudaStream_t s) {
 extern "C" {
 
 static int create_engine(const b2sd_config* cfg, std::shared_ptr<WeightStore> store, b2sd_handle* out);
+static int alloc_unet_rows(b2sd_handle e, int rows);
 
 int b2sd_create(const b2sd_config* cfg, b2sd_handle* out) { return create_engine(cfg, std::make_shared<WeightStore>(), out); }
 
@@ -1202,20 +1247,18 @@ static int create_engine(const b2sd_config* cfg, std::shared_ptr<WeightStore> st
     e->cfg = *cfg;
     e->lh = cfg->height / 8;
     e->lw = cfg->width / 8;
-    const int B = cfg->batch, C0 = cfg->block_out_channels[0];
+    const int B = cfg->batch;
     e->x_in.n = B; e->x_in.h = e->lh; e->x_in.w = e->lw; e->x_in.c = 4; e->x_in.ld = 4;
     e->x_in.p = static_cast<__half*>(e->state.alloc((size_t)e->x_in.elems() * 2));
     e->noise = static_cast<__half*>(e->state.alloc((size_t)e->x_in.elems() * 2));
+    e->stock = static_cast<__half*>(e->state.alloc((size_t)e->x_in.elems() * 2));
     e->coef = static_cast<float*>(e->state.alloc(4 * B * sizeof(float)));
-    e->tsteps = static_cast<float*>(e->state.alloc(B * sizeof(float)));
     e->ctx = static_cast<__half*>(e->state.alloc((size_t)cfg->ctx_tokens * cfg->cross_attention_dim * 2));
-    e->temb_sin = static_cast<float*>(e->state.alloc((size_t)B * C0 * sizeof(float)));
-    e->temb_h = static_cast<float*>(e->state.alloc((size_t)B * 4 * C0 * sizeof(float)));
-    e->temb = static_cast<float*>(e->state.alloc((size_t)B * 4 * C0 * sizeof(float)));
-    e->gn_ws = static_cast<float*>(e->state.alloc(groupnorm_partial_floats(B, cfg->norm_groups) * sizeof(float)));
+    e->uctx = static_cast<__half*>(e->state.alloc((size_t)cfg->ctx_tokens * cfg->cross_attention_dim * 2));
     e->tile_counters = static_cast<int*>(e->state.alloc(65536 * sizeof(int)));
     if (e->tile_counters) cudaMemset(e->tile_counters, 0, 65536 * sizeof(int));
-    if (!e->x_in.p || !e->noise || !e->coef || !e->tsteps || !e->ctx || !e->temb || !e->gn_ws) {
+    if (e->stock) cudaMemset(e->stock, 0, (size_t)e->x_in.elems() * 2);
+    if (!e->x_in.p || !e->noise || !e->stock || !e->coef || !e->ctx || !e->uctx || alloc_unet_rows(e, B)) {
         b2_set_error("b2sd_create: cudaMalloc failed");
         delete e;
         return -1;
@@ -1298,8 +1341,35 @@ int b2sd_load_tensor(b2sd_handle h, const char* key, const void* ptr, int dtype,
     return 0;
 }
 
+// Per-UNet-row state (timesteps, time embeddings, GroupNorm workspace) for `rows` rows; grows only (bump arena).
+static int alloc_unet_rows(b2sd_handle e, int rows) {
+    if (rows <= e->rows_cap) return 0;
+    const int C0 = e->cfg.block_out_channels[0];
+    e->tsteps = static_cast<float*>(e->state.alloc(rows * sizeof(float)));
+    e->temb_sin = static_cast<float*>(e->state.alloc((size_t)rows * C0 * sizeof(float)));
+    e->temb_h = static_cast<float*>(e->state.alloc((size_t)rows * 4 * C0 * sizeof(float)));
+    e->temb = static_cast<float*>(e->state.alloc((size_t)rows * 4 * C0 * sizeof(float)));
+    e->gn_ws = static_cast<float*>(e->state.alloc(groupnorm_partial_floats(rows, e->cfg.norm_groups) * sizeof(float)));
+    if (!e->tsteps || !e->temb_sin || !e->temb_h || !e->temb || !e->gn_ws) {
+        b2_set_error("cudaMalloc of the per-row UNet state (%d rows) failed", rows);
+        return -1;
+    }
+    e->rows_cap = rows;
+    return 0;
+}
+
+// sub_timesteps [T] -> tsteps of the UNet rows: row r < uc_rows takes t[r], row r >= uc_rows takes t[r - uc_rows]
+static int upload_timesteps(b2sd_handle h, const float* timesteps, cudaStream_t s) {
+    const int rows = h->unet_rows(), u = h->uc_rows;
+    std::vector<float> t(rows);
+    for (int r = 0; r < rows; ++r) t[r] = timesteps[r < u ? r : r - u];
+    CUDA_OK(cudaMemcpyAsync(h->tsteps, t.data(), rows * sizeof(float), cudaMemcpyHostToDevice, s));
+    CUDA_OK(cudaStreamSynchronize(s));
+    return 0;
+}
+
 static int refresh_time(b2sd_handle h, cudaStream_t s) {
-    const int B = h->cfg.batch, C0 = h->cfg.block_out_channels[0], TD = 4 * C0;
+    const int B = h->unet_rows(), C0 = h->cfg.block_out_channels[0], TD = 4 * C0;
     const Raw* w1 = h->get("time_embedding.linear_1.weight");
     const Raw* w2 = h->get("time_embedding.linear_2.weight");
     const float* b1 = h->vec({"time_embedding.linear_1.bias"});
@@ -1319,12 +1389,29 @@ int b2sd_prepare(b2sd_handle h, const void* prompt_embeds, const float* timestep
     }
     cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
     const int B = h->cfg.batch, lh = h->lh, lw = h->lw;
+    // guidance requested by b2sd_set_guidance takes effect here
+    const b2sd_engine::Guidance& g = h->guide_req;
+    const bool guided = g.cfg_type != B2SD_CFG_NONE && g.scale > 1.f;
+    const int uc = !guided ? 0 : (g.cfg_type == B2SD_CFG_INITIALIZE ? 1 : (g.cfg_type == B2SD_CFG_FULL ? B : 0));
+    if (B + uc > 16) {
+        b2_set_error("b2sd_prepare: the guided UNet batch of %d rows exceeds 16", B + uc);
+        return -1;
+    }
+    if (uc > 0 && h->uncond_host.empty()) {
+        b2_set_error("b2sd_prepare: cfg_type initialize / full needs the unconditional embeddings (b2sd_set_guidance)");
+        return -1;
+    }
+    TRY(alloc_unet_rows(h, B + uc));
+    h->guide = guided ? g : b2sd_engine::Guidance{};
+    h->uc_rows = uc;
     for (int k = 0; k < 4; ++k)
         for (int i = 0; i < B; ++i) h->coef_host[k][i] = coef[k * B + i];
     CUDA_OK(cudaMemcpyAsync(h->coef, coef, 4 * B * sizeof(float), cudaMemcpyHostToDevice, s));
-    CUDA_OK(cudaMemcpyAsync(h->tsteps, timesteps, B * sizeof(float), cudaMemcpyHostToDevice, s));
+    TRY(upload_timesteps(h, timesteps, s));
     CUDA_OK(cudaMemcpyAsync(h->ctx, prompt_embeds, (size_t)h->cfg.ctx_tokens * h->cfg.cross_attention_dim * 2,
                             cudaMemcpyHostToDevice, s));
+    if (uc > 0)
+        CUDA_OK(cudaMemcpyAsync(h->uctx, h->uncond_host.data(), h->uncond_host.size() * 2, cudaMemcpyHostToDevice, s));
     // init_noise NCHW -> NHWC (host side; once per prepare)
     {
         const __half* src = static_cast<const __half*>(init_noise);
@@ -1337,8 +1424,9 @@ int b2sd_prepare(b2sd_handle h, const void* prompt_embeds, const float* timestep
         CUDA_OK(cudaMemcpyAsync(h->noise, nhwc.data(), nhwc.size() * 2, cudaMemcpyHostToDevice, s));
         CUDA_OK(cudaStreamSynchronize(s));
     }
-    // x_t_latent_buffer = zeros (StreamDiffusion.prepare); slot 0 is overwritten by every frame
+    // x_t_latent_buffer = zeros, stock_noise = zeros (StreamDiffusion.prepare); slot 0 is overwritten by every frame
     CUDA_OK(cudaMemsetAsync(h->x_in.p, 0, (size_t)h->x_in.elems() * 2, s));
+    CUDA_OK(cudaMemsetAsync(h->stock, 0, (size_t)h->x_in.elems() * 2, s));
     TRY(h->build_program(s));
     TRY(h->run(h->prog_prompt, s));
     TRY(refresh_time(h, s));
@@ -1522,9 +1610,28 @@ int b2sd_set_timesteps(b2sd_handle h, const float* timesteps, void* stream) {
         return -1;
     }
     cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-    CUDA_OK(cudaMemcpyAsync(h->tsteps, timesteps, h->cfg.batch * sizeof(float), cudaMemcpyHostToDevice, s));
-    CUDA_OK(cudaStreamSynchronize(s));
+    TRY(upload_timesteps(h, timesteps, s));
     return refresh_time(h, s);
+}
+
+int b2sd_set_guidance(b2sd_handle h, int cfg_type, float guidance_scale, float delta, const void* uncond_embeds) {
+    if (!h || cfg_type < B2SD_CFG_NONE || cfg_type > B2SD_CFG_FULL) {
+        b2_set_error("b2sd_set_guidance: bad argument (cfg_type %d)", cfg_type);
+        return -1;
+    }
+    if ((cfg_type == B2SD_CFG_INITIALIZE || cfg_type == B2SD_CFG_FULL) && guidance_scale > 1.f && !uncond_embeds) {
+        b2_set_error("b2sd_set_guidance: cfg_type initialize / full needs the unconditional prompt embeddings");
+        return -1;
+    }
+    h->guide_req.cfg_type = cfg_type;
+    h->guide_req.scale = guidance_scale;
+    h->guide_req.delta = delta;
+    if (uncond_embeds) {
+        const __half* src = static_cast<const __half*>(uncond_embeds);
+        h->uncond_host.assign(src, src + (size_t)h->cfg.ctx_tokens * h->cfg.cross_attention_dim);
+    }
+    h->built = false;   // applied when the frame program is built (b2sd_prepare)
+    return 0;
 }
 
 int b2sd_step(b2sd_handle h, const void* frame_in, int in_h, int in_w, void* frame_out, void* stream) {
@@ -1765,6 +1872,7 @@ int b2sd_share_stream_state(b2sd_handle lane, b2sd_handle owner) {
     }
     lane->group = owner->group;
     lane->x_in.p = owner->x_in.p;        // the UNet input batch: slot 0 = fresh x_t, slots 1.. = x_t_latent_buffer
+    lane->stock = owner->stock;          // stock_noise of residual guidance
     lane->built = false;
     owner->built = false;
     return 0;

@@ -71,6 +71,8 @@ IG_RELU = 1
 IG_GEGLU = 2
 IG_TCONV = 64
 IG_PAIR = 128
+CFG_NONE, CFG_SELF, CFG_INITIALIZE, CFG_FULL = 0, 1, 2, 3
+CFG_TYPES = {"none": CFG_NONE, "self": CFG_SELF, "initialize": CFG_INITIALIZE, "full": CFG_FULL}
 
 _lib = None
 
@@ -100,6 +102,7 @@ def lib() -> C.CDLL:
         _lib.b2sd_op_upsample2x.argtypes = [vp, vp, ci, ci, ci, ci, vp]
         _lib.b2sd_op_smallconv.argtypes = [vp, vp, vp, vp, ci, ci, ci, ci, ci, ci, ci, ci, ci, vp]
         _lib.b2sd_op_lcm_step.argtypes = [vp, vp, vp, vp, vp, ci, ci, ci, vp]
+        _lib.b2sd_op_lcm_cfg_step.argtypes = [vp, vp, vp, vp, vp, vp, ci, ci, ci, ci, cf, cf, vp]
         _lib.b2sd_op_post_u8.argtypes = [vp, ci, vp, ci, ci, ci, vp]
         _lib.b2sd_op_nv12_to_rgb.argtypes = [vp, ci, vp, ci, vp, ci, ci, ci, vp]
         _lib.b2sd_op_rgb_to_nv12.argtypes = [vp, vp, ci, vp, ci, ci, ci, ci, vp]
@@ -113,6 +116,7 @@ def lib() -> C.CDLL:
         _lib.b2sd_import_packed.argtypes = [vp, C.c_char_p]
         _lib.b2sd_set_prompt_embeds.argtypes = [vp, vp, vp]
         _lib.b2sd_set_timesteps.argtypes = [vp, vp, vp]
+        _lib.b2sd_set_guidance.argtypes = [vp, ci, cf, cf, vp]
         _lib.b2sd_step.argtypes = [vp, vp, ci, ci, vp, vp]
         _lib.b2sd_step_ex.argtypes = [vp, vp, ci, ci, ci, vp, ci, vp]
         _lib.b2sd_get_tensor.argtypes = [vp, C.c_char_p, vp, i64, C.POINTER(i64), C.POINTER(ci), vp]
@@ -127,10 +131,11 @@ def lib() -> C.CDLL:
         _lib.b2sd_profile_kind.restype = C.c_int
         _lib.b2sd_profile_gate.argtypes = [ci]
         _lib.b2sd_profile_gate.restype = C.c_int
-        for name in ("create", "create_lane", "destroy", "load_tensor", "prepare", "export_packed", "import_packed", "set_prompt_embeds", "set_timesteps", "step",
+        for name in ("create", "create_lane", "destroy", "load_tensor", "prepare", "export_packed", "import_packed", "set_prompt_embeds", "set_timesteps",
+                     "set_guidance", "step",
                      "step_ex", "get_tensor", "launches_per_step"):
             getattr(_lib, "b2sd_" + name).restype = C.c_int
-        for name in ("attention", "groupnorm", "layernorm", "upsample2x", "smallconv", "lcm_step", "post_u8", "nv12_to_rgb", "rgb_to_nv12"):
+        for name in ("attention", "groupnorm", "layernorm", "upsample2x", "smallconv", "lcm_step", "lcm_cfg_step", "post_u8", "nv12_to_rgb", "rgb_to_nv12"):
             getattr(_lib, "b2sd_op_" + name).restype = C.c_int
     return _lib
 

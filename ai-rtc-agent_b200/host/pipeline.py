@@ -56,12 +56,16 @@ def _as_torch_u8_nhwc(frame, device) -> torch.Tensor:
 
 class StreamDiffusionPipeline:
     def __init__(self, model_id: str, t_index_list: Optional[List[int]] = None, width: int = 512, height: int = 512,
-                 prompt: str = DEFAULT_PROMPT, lanes: Optional[int] = None):
+                 prompt: str = DEFAULT_PROMPT, lanes: Optional[int] = None, *, cfg_type: str = "self",
+                 guidance_scale: float = DEFAULT_GUIDANCE_SCALE, delta: float = 1.0, negative_prompt: str = ""):
         """lanes: frames in flight for enqueue() ($B200SD_LANES overrides the default).  With a 1-step stream batch (SD-Turbo)
         consecutive frames are independent: DEFAULT_LANES_ONE_STEP lanes process frame n+1.. while frame n is still on the GPU.
         With T > 1 the stream batch carries state from frame to frame: two lanes share that state and are stage-pipelined (TAESD
         encoder of frame n+1 and decoder of frame n-1 overlap the UNet of frame n).  Both are bit-identical to submitting the
-        same frames one at a time."""
+        same frames one at a time.
+        cfg_type / guidance_scale / delta / negative_prompt: StreamDiffusion's classifier-free guidance (active when
+        guidance_scale > 1 and cfg_type != "none"); the defaults are unguided.  Residual guidance ("self") carries its stock
+        noise from frame to frame even with a 1-step stream batch, so such a stream runs on two shared-state lanes too."""
         self.prompt = prompt
         self.t_index_list = list(t_index_list) if t_index_list is not None else DEFAULT_T_INDEX_LIST
         self.device = "cuda"
@@ -78,10 +82,11 @@ class StreamDiffusionPipeline:
             mode="img2img",
             use_denoising_batch=True,
             use_tiny_vae=True,
-            cfg_type="self",
+            cfg_type=cfg_type,
             engine_dir=os.getenv("TRT_ENGINES_CACHE", "./models/engines"),
         )
-        stateful = len(self.t_index_list) > 1     # x_t_latent_buffer chains frame n+1 to frame n
+        # x_t_latent_buffer (T > 1) or the stock noise of residual guidance chains frame n+1 to frame n
+        stateful = len(self.t_index_list) > 1 or (cfg_type == "self" and guidance_scale > 1.0)
         if lanes is None:
             lanes = int(os.getenv("B200SD_LANES", "0")) or (DEFAULT_LANES_STATEFUL if stateful else DEFAULT_LANES_ONE_STEP)
         if stateful:
@@ -89,8 +94,8 @@ class StreamDiffusionPipeline:
         # launch policy = number of frames in flight ($B200SD_POLICY_FRAMES overrides it for profiling: a single lane running the
         # throughput policy's launches gives ncu a clean one-frame launch list)
         self.model.stream.set_concurrency(max(1, int(os.environ.get("B200SD_POLICY_FRAMES", lanes))))
-        self.model.prepare(prompt=self.prompt, num_inference_steps=DEFAULT_NUM_INFERENCE_STEPS,
-                           guidance_scale=DEFAULT_GUIDANCE_SCALE)
+        self.model.prepare(prompt=self.prompt, negative_prompt=negative_prompt, num_inference_steps=DEFAULT_NUM_INFERENCE_STEPS,
+                           guidance_scale=guidance_scale, delta=delta)
         sd = self.model.stream
         self._engines = [sd] + [sd.add_lane(share_state=stateful) for _ in range(max(1, lanes) - 1)]
         # one lane: frames run on the caller's stream, exactly as before.  Several lanes: every lane has its own stream (a lane on

@@ -3,8 +3,8 @@ yondonfu/StreamDiffusion@deepstream), re-implemented over libb200sd.so: the host
 (LCM timestep table, per-slot scalars, seeded noise, prompt embedding, attributes that
 lib/wrapper.py:389-407 pokes at) lives here in Python, everything per-frame runs in the engine.
 
-Supported configuration = the one lib/pipeline.py:23-42 builds: img2img, use_denoising_batch=True,
-frame_buffer_size=1, cfg_type "self"/"none" with guidance_scale <= 1.0 (no CFG arithmetic)."""
+Supported configuration: img2img, use_denoising_batch=True, frame_buffer_size=1, every cfg_type ("none", "self",
+"initialize", "full") at any guidance_scale (lib/pipeline.py:23-42 builds "self" with guidance 0.0, i.e. no guidance)."""
 from __future__ import annotations
 
 import ctypes as C
@@ -44,6 +44,12 @@ def lcm_boundary_scalings(timestep: int):
     scaled = timestep * LCM_TIMESTEP_SCALING
     denom = scaled * scaled + LCM_SIGMA_DATA * LCM_SIGMA_DATA
     return LCM_SIGMA_DATA * LCM_SIGMA_DATA / denom, scaled / denom ** 0.5
+
+
+def uncond_rows(cfg_type: str, frame_buffer_size: int, batch_size: int) -> int:
+    """Unconditional rows a guided UNet batch puts in front of the batch_size text rows (upstream StreamDiffusion.__init__'s
+    trt_unet_batch_size): one per frame for "initialize", one per text row for "full", none for "self" / "none"."""
+    return {"initialize": frame_buffer_size, "full": batch_size}.get(cfg_type, 0)
 
 
 class ImageProcessor:
@@ -92,7 +98,11 @@ class StreamDiffusion:
         self.cfg_type = cfg_type
         self.use_denoising_batch = use_denoising_batch
         self.batch_size = self.denoising_steps_num * frame_buffer_size
-        self.trt_unet_batch_size = self.batch_size  # cfg "self"/"none": no extra unconditional rows
+        # UNet batch of a guided stream (StreamDiffusion.__init__): initialize adds one unconditional row, full T of them.
+        # prepare() sets it to the batch the engine actually runs (T when guidance is off).
+        self.trt_unet_batch_size = self.batch_size + uncond_rows(cfg_type, frame_buffer_size, self.batch_size)
+        self._uc_rows = 0
+        self._uncond: Optional[torch.Tensor] = None
         self.t_list = list(t_index_list)
         self.do_add_noise = do_add_noise
         self.similar_image_filter = False
@@ -185,12 +195,16 @@ class StreamDiffusion:
         self.generator = generator if generator is not None else torch.Generator()
         self.generator.manual_seed(seed)
         self.guidance_scale = 1.0 if self.cfg_type == "none" else guidance_scale
-        if self.guidance_scale > 1.0:
-            raise NotImplementedError("classifier-free guidance (guidance_scale > 1) is not on the reference's path "
-                                      "(lib/pipeline.py:14 passes 0.0)")
         self.delta = delta
         T = self.denoising_steps_num
-        self.prompt_embeds = self._encode(prompt).repeat(self.batch_size, 1, 1)
+        guided = self.guidance_scale > 1.0
+        cond = self._encode(prompt)
+        self._uc_rows = uncond_rows(self.cfg_type, self.frame_bff_size, self.batch_size) if guided else 0
+        # residual guidance ("self") needs no negative prompt: its unconditional prediction is delta * stock_noise
+        self._uncond = self._encode(negative_prompt) if self._uc_rows else None
+        self.trt_unet_batch_size = self.batch_size + self._uc_rows
+        # uncond-first layout: initialize [uncond, cond x T], full [uncond x T, cond x T], otherwise [cond x T]
+        self.prompt_embeds = self._embeds_rows(cond)
         self.timesteps = lcm_timestep_table(num_inference_steps)
         self.sub_timesteps = [self.timesteps[t] for t in self.t_list]
         self.sub_timesteps_tensor = torch.tensor(self.sub_timesteps, dtype=torch.long, device=self.device)
@@ -210,14 +224,24 @@ class StreamDiffusion:
             lane._prepare_like(self)
 
     _SCHEDULE_ATTRS = ("generator", "guidance_scale", "delta", "prompt_embeds", "timesteps", "sub_timesteps", "sub_timesteps_tensor",
-                       "init_noise", "stock_noise", "c_skip", "c_out", "alpha_prod_t_sqrt", "beta_prod_t_sqrt")
+                       "init_noise", "stock_noise", "c_skip", "c_out", "alpha_prod_t_sqrt", "beta_prod_t_sqrt", "trt_unet_batch_size",
+                       "_uc_rows", "_uncond")
+
+    def _embeds_rows(self, cond: torch.Tensor) -> torch.Tensor:
+        rows = cond.repeat(self.batch_size, 1, 1)
+        if self._uc_rows:
+            rows = torch.cat([self._uncond.repeat(self._uc_rows, 1, 1), rows], dim=0)
+        return rows
 
     def _engine_prepare(self) -> None:
         coef = torch.stack([self.alpha_prod_t_sqrt.flatten(), self.beta_prod_t_sqrt.flatten(),
                             self.c_skip.flatten(), self.c_out.flatten()]).float().contiguous()
         tsteps = torch.tensor(self.sub_timesteps, dtype=torch.float32)
-        emb = self.prompt_embeds[0].to(torch.float16).cpu().contiguous()
+        emb = self.prompt_embeds[self._uc_rows].to(torch.float16).cpu().contiguous()
         noise = self.init_noise.cpu().contiguous()
+        unc = self._uncond[0].to(torch.float16).cpu().contiguous() if self._uncond is not None else None
+        capi.check(self._lib.b2sd_set_guidance(self._handle, capi.CFG_TYPES[self.cfg_type], float(self.guidance_scale),
+                                               float(self.delta), None if unc is None else unc.data_ptr()), "b2sd_set_guidance")
         capi.check(self._lib.b2sd_prepare(self._handle, emb.data_ptr(), tsteps.data_ptr(), coef.data_ptr(),
                                           noise.data_ptr(), self._stream()), "b2sd_prepare")
         self._prepared = True
@@ -254,8 +278,12 @@ class StreamDiffusion:
 
     @torch.no_grad()
     def update_prompt(self, prompt: str) -> None:
-        self.prompt_embeds = self._encode(prompt).repeat(self.batch_size, 1, 1)
-        emb = self.prompt_embeds[0].cpu().contiguous()
+        """Replaces the conditional rows only.  Upstream StreamDiffusion.update_prompt re-encodes the prompt into batch_size
+        rows and so drops the unconditional rows of an initialize / full batch, which then no longer matches the UNet batch;
+        here those rows keep the negative prompt of prepare() (a deliberate deviation)."""
+        cond = self._encode(prompt)
+        self.prompt_embeds = self._embeds_rows(cond)
+        emb = cond[0].cpu().contiguous()
         for eng in [self] + self.lanes:
             eng.prompt_embeds = self.prompt_embeds
             capi.check(self._lib.b2sd_set_prompt_embeds(eng._handle, emb.data_ptr(), self._stream()), "b2sd_set_prompt_embeds")

@@ -16,7 +16,7 @@ import torch
 from PIL import Image
 
 from .prompt import make_prompt_encoder
-from .stream import StreamDiffusion
+from .stream import StreamDiffusion, uncond_rows
 from .weights import resolve_weights
 
 logger = logging.getLogger(__name__)
@@ -103,8 +103,6 @@ class StreamDiffusionWrapper:
             unsupported.append("DataParallel device_ids (shard streams across GPUs instead, see host/dist.py)")
         if not use_tiny_vae:
             unsupported.append("full AutoencoderKL (only TAESD is on the reference's path)")
-        if cfg_type in ("full", "initialize"):
-            unsupported.append(f"cfg_type='{cfg_type}'")
         if device != "cuda":
             unsupported.append("device='cpu' (no CPU fallback)")
         if unsupported:
@@ -154,7 +152,7 @@ class StreamDiffusionWrapper:
         if use_cache:
             blob = W.packed_blob_path(self.engine_dir, model_id_or_path, arch.name, use_lcm_lora and not self.sd_turbo, lcm_lora_id,
                                       lora_dict, vae_id, synthetic=not have_ckpt,
-                                      variant=W.layout_variant(self.batch_size, self.height, self.width))
+                                      variant=W.layout_variant(self._unet_batch(cfg_type), self.height, self.width))
         encoder = make_prompt_encoder(repo if have_ckpt else None, arch.cross_attention_dim, self.device, allow_synthetic=synthetic_ok)
         if blob is not None and os.path.exists(blob) and (have_ckpt or synthetic_ok):
             try:
@@ -168,6 +166,11 @@ class StreamDiffusionWrapper:
                                                       self.sd_turbo)
         self._blob_to_write = blob
         return StreamDiffusion(arch, unet_sd, vae_sd, t_index_list, encoder, **kw)
+
+    def _unet_batch(self, cfg_type: str) -> int:
+        """UNet batch of a guided stream: initialize adds one unconditional row per frame, full one per stream-batch row.  The
+        packed layout is chosen for it (those cfg types are used with guidance_scale > 1)."""
+        return self.batch_size + uncond_rows(cfg_type, self.frame_buffer_size, self.batch_size)
 
     def _on_stream(self):
         return torch.cuda.stream(self._ext_stream) if self._ext_stream is not None else _NullCtx()

@@ -136,6 +136,14 @@ int b2sd_op_smallconv(const void* x, const void* w_oihw, const float* bias, void
 /* StreamDiffusion scheduler_step_batch + stream-batch buffer update (see elementwise.cuh) */
 int b2sd_op_lcm_step(void* x, const void* eps, const void* noise, const float* coef, void* out_latent, int T,
                      int hw, int do_add_noise, void* stream);
+/* Classifier-free guidance types of StreamDiffusion (cfg_type "none" / "self" / "initialize" / "full") */
+enum { B2SD_CFG_NONE = 0, B2SD_CFG_SELF = 1, B2SD_CFG_INITIALIZE = 2, B2SD_CFG_FULL = 3 };
+/* The same step with residual / full classifier-free guidance (StreamDiffusion.unet_step with guidance_scale > 1), fused:
+ * eps = UNet output rows, unconditional rows first (0 for self, 1 for initialize, T for full, then T text rows);
+ * stock_noise fp16 [T][hw][4] is read and updated in place.  cfg_type is B2SD_CFG_SELF / _INITIALIZE / _FULL
+ * (see elementwise.cuh for the arithmetic). */
+int b2sd_op_lcm_cfg_step(void* x, const void* eps, const void* noise, void* stock_noise, const float* coef, void* out_latent,
+                         int T, int hw, int do_add_noise, int cfg_type, float guidance_scale, float delta, void* stream);
 /* Codec boundary (SURVEY.md 8f-1; the reference's aiortc fork decodes with NVDEC / encodes with NVENC, requirements.txt:12-13,
  * and exchanges RGB tensors in HBM with lib/pipeline.py:50-51,83,96).  NV12 surface (Y plane + interleaved UV plane, pitches in
  * bytes) <-> the frame formats of b2sd_step: u8 NHWC RGB in, u8 NCHW RGB out.  flags: 0 = BT.709 limited range,
@@ -151,7 +159,7 @@ int b2sd_op_post_u8(const void* y_nhwc, int ldy, void* out_nchw_u8, int nb, int 
  * Engine level: one handle == one temporal stream (one StreamDiffusion instance, lib/wrapper.py:168).
  * Replaces StreamDiffusion + UNet2DConditionModelEngine + AutoencoderKLEngine
  * (lib/wrapper.py:445-466, 494-504) for mode="img2img", use_denoising_batch=True, frame_buffer_size=1,
- * cfg_type="self" with guidance_scale <= 1 (the only configuration lib/pipeline.py:23-42 builds).
+ * cfg_type "none" / "self" / "initialize" / "full" (b2sd_set_guidance; lib/pipeline.py:23-42 builds "self" with guidance 0).
  * ---------------------------------------------------------------------------------------------- */
 typedef struct b2sd_engine* b2sd_handle;
 
@@ -205,10 +213,20 @@ int b2sd_import_packed(b2sd_handle h, const char* path);
  * Synchronises `stream`. */
 int b2sd_prepare(b2sd_handle h, const void* prompt_embeds, const float* timesteps, const float* coef,
                  const void* init_noise, void* stream);
-/* StreamDiffusion.update_prompt (lib/pipeline.py:44-45): refresh the per-layer cross-attention K/V cache */
+/* Classifier-free guidance of StreamDiffusion.prepare (guidance_scale, delta, cfg_type, negative_prompt).  Takes effect at the
+ * next b2sd_prepare, like b2sd_set_concurrency.  Guidance is active when cfg_type != B2SD_CFG_NONE and guidance_scale > 1;
+ * otherwise the frame program is the unguided one.  Active guidance runs the UNet on B_u rows: T (self), T + 1 (initialize:
+ * [uncond slot 0 | T text rows]) or 2T (full: [T uncond | T text]), and keeps stock_noise [T][h/8][w/8][4] in the stream
+ * state (zeroed by b2sd_prepare, shared by b2sd_share_stream_state, tap "stock_noise").  uncond_embeds: HOST fp16
+ * [ctx_tokens][cross_attention_dim], the encoded negative prompt; required for initialize / full, may be NULL otherwise.
+ * B_u must not exceed 16. */
+int b2sd_set_guidance(b2sd_handle h, int cfg_type, float guidance_scale, float delta, const void* uncond_embeds);
+/* StreamDiffusion.update_prompt (lib/pipeline.py:44-45): refresh the per-layer cross-attention K/V cache.  Replaces the
+ * conditional prompt only; the unconditional rows of a guided batch keep the negative prompt of b2sd_set_guidance. */
 int b2sd_set_prompt_embeds(b2sd_handle h, const void* prompt_embeds, void* stream);
 /* lib/wrapper.py:389-407 update_t_index_list: only sub_timesteps change (alpha/beta/c_skip/c_out keep the
- * values given to b2sd_prepare -- reference behaviour) */
+ * values given to b2sd_prepare -- reference behaviour).  timesteps: fp32 [batch]; the engine repeats them for the extra
+ * unconditional rows of a guided UNet batch. */
 int b2sd_set_timesteps(b2sd_handle h, const float* timesteps, void* stream);
 
 /* One StreamDiffusionPipeline.__call__ (lib/pipeline.py:76-96, NVENC branch): frame_in = device u8 NHWC
@@ -225,7 +243,7 @@ int b2sd_step_ex(b2sd_handle h, const void* frame_in, int in_kind, int in_h, int
                  int out_kind, void* stream);
 
 /* Parity/debug taps: copies a named intermediate of the last step to host memory as fp16 NHWC.
- * Names: "x_t", "unet_in", "eps", "x0", "image", "conv_in", "down.I.J", "mid", "up.I.J".
+ * Names: "x_t", "unet_in", "eps" (all B_u UNet rows), "x0", "image", "conv_in", "down.I.J", "mid", "up.I.J", "stock_noise".
  * Returns the element count via *count (pass dst = NULL to query).  Synchronises `stream`. */
 int b2sd_get_tensor(b2sd_handle h, const char* name, void* dst, int64_t capacity, int64_t* count, int* dims4,
                     void* stream);
